@@ -2,11 +2,13 @@
 """Benchmark of the hot path BASELINE.json names: ItemKNN cosine top-K rows/sec (and BPR samples/sec as a
 secondary figure) on a synthetic CSR URM.
 
-    python bench.py --gpus N --steps K --warmup W [--impl b200|reference] [--workload C5]
+    python bench.py --gpus N --steps K --warmup W [--impl b200|reference] [--workload C5] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one full pass of the similarity hot path over the workload
 (all n_items columns: accumulate + normalise + top-K, plus the all-gather when N > 1) with the URM already
-resident in HBM.  `e2e` is the same metric through the reference-facing Python call
+resident in HBM.  `--dump-outputs DIR` writes the top-K table of the last timed step to DIR (dump_topk_table) so that
+two builds can be compared output for output; the URM is generated from a fixed seed, so the inputs are the same in
+every run with the same arguments.  `e2e` is the same metric through the reference-facing Python call
 (Compute_Similarity_Cython(URM, ...).compute_similarity() -> scipy CSR) with HOST buffers: H2D of the CSR,
 device-side constructor work, kernel, CSR assembly and D2H all inside the timed region.
 
@@ -255,6 +257,30 @@ def parity_gate(X, table, W_ref, lo, hi, K, kind):
     return res
 
 
+DUMP_COLS = 16384  # at K = 200: 16384 x 200 x (8 + 4) B = 39 MB of neighbour ids and values
+
+
+def dump_topk_table(path, table):
+    """Writes the [n_items, K] top-K table (idx, val, cnt) as path/<name>.npy for a fixed, seeded sample of DUMP_COLS target
+    columns (all of them when there are fewer): columns.npy (the sampled target columns), neighbours.npy and similarities.npy
+    ([columns, K]) and counts.npy.  The kernel's slot order within a column is unspecified, so each column's entries are put
+    in ascending neighbour order -- the order of a column of the CSR matrix compute_similarity() returns -- with the unused
+    slots (at and beyond counts) last, as neighbour -1 and similarity 0.  Ids are stored as float64, which holds them exactly."""
+    import torch
+    idx, val, cnt = table
+    n, K = idx.shape
+    cols = np.arange(n) if n <= DUMP_COLS else np.sort(np.random.default_rng(0).choice(n, DUMP_COLS, replace=False))
+    sel = torch.from_numpy(cols).to(idx.device)
+    i, v, c = (t.index_select(0, sel).cpu().numpy() for t in (idx, val, cnt))
+    unused = np.arange(K)[None, :] >= c[:, None]
+    i, v = np.where(unused, -1, i), np.where(unused, 0.0, v)
+    order = np.argsort(np.where(unused, np.iinfo(np.int64).max, i.astype(np.int64)), axis=1, kind="stable")
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("columns", cols.astype(np.float64)), ("neighbours", np.take_along_axis(i, order, 1).astype(np.float64)),
+                    ("similarities", np.take_along_axis(v, order, 1).astype(np.float32)), ("counts", c.astype(np.float64))):
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------------------
 def pinned_csr(X):
     """scipy CSR whose three arrays live in pinned host memory (so the e2e H2D runs at PCIe speed)."""
@@ -345,6 +371,8 @@ def run_b200(args, rank, world, local_rank):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         elapsed_ms = float(t.item())
     value = n_items * args.steps / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_topk_table(args.dump_outputs, out)
 
     # ---- kernel-only roofline leg (CUDA events around the kernel on its launching stream, inside the library)
     kms = []
@@ -504,7 +532,7 @@ def bpr_leg_sharded(args, X, rank, world):
         tr.flush()
         torch.cuda.synchronize(); dist.barrier()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        steps = max(10, args.steps)
+        steps = args.steps
         ev0.record()
         n = 0
         for _ in range(steps):
@@ -549,7 +577,7 @@ def bpr_leg(args, X):
             m.epochIteration_Cython()
         torch.cuda.synchronize()
         walls, devs = [], []
-        for _ in range(max(3, args.steps)):
+        for _ in range(args.steps):
             t = time.perf_counter()
             m.epochIteration_Cython()
             torch.cuda.synchronize()
@@ -601,7 +629,7 @@ def bpr_leg(args, X):
                 m.epochIteration_Cython()
             torch.cuda.synchronize()
             devs = []
-            for _ in range(10):
+            for _ in range(args.steps):
                 m.epochIteration_Cython()
                 torch.cuda.synchronize()
                 devs.append(m.last_epoch_ms() * 1e-3)
@@ -704,7 +732,12 @@ def main():
     ap.add_argument("--ref-workers", type=int, default=64, help="worker processes of the reference arm (capped by the host core count)")
     ap.add_argument("--ref-slice", type=int, default=250)
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"], help="N > 1: how the ranks' rows reach every rank")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the top-K table of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the output of --impl b200; the reference arm times column slices and keeps no output")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

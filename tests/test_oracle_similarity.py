@@ -131,35 +131,35 @@ def test_euclidean_oracle_dense_control():
     assert np.allclose(S, ctrl, atol=1e-6)
 
 
-@pytest.mark.skipif(ref_loader.load("Compute_Similarity_Cython") is None, reason="oracle/_ref not built")
 def test_reference_comparer_on_tied_binary_data():
-    """compare_topk_with_reference (bench.py's parity gate) accepts the oracle's result against the compiled reference on
-    binary data, where the K boundary is full of ties the two resolve differently, and rejects corrupted results."""
+    """compare_topk_with_reference (bench.py's parity gate) accepts the oracle's result against the compiled reference's
+    own output (stored in similarity_golden.npz) on binary data, where the K boundary is full of ties the two resolve
+    differently, and rejects corrupted results."""
     from oracle.similarity_oracle import compare_topk_with_reference, cosine_pair_values
-    cy = ref_loader.load("Compute_Similarity_Cython").Compute_Similarity_Cython
-    X = synth_urm(1500, 300, 0.04, seed=9, values="binary")
-    kw = dict(topK=15, shrink=10, similarity="cosine")
-    Wr = cy(X, **kw).compute_similarity()
+    values, kw, W = CASES[16]
+    assert values == "binary" and kw["similarity"] == "cosine"
+    X, K, n = URMS[values], kw["topK"], 150
+    Wr = W["cy"]
     Wo = SimilarityOracle(X, **kw).compute_similarity()
     Xc = sps.csc_matrix(X)
-    pv = lambda jj, cc: cosine_pair_values(Xc, jj, cc, 10)
-    res = compare_topk_with_reference(Wo, Wr, np.arange(300), 15, pair_values=pv)
+    pv = lambda jj, cc: cosine_pair_values(Xc, jj, cc, kw["shrink"])
+    res = compare_topk_with_reference(Wo, Wr, np.arange(n), K, pair_values=pv)
     assert res["ok"], res
     assert res["tie_cols"] > 0 and res["tie_pairs_checked"] > 0  # the case really exercises the tie path
     # a wrong value on one entry
     bad = sps.csc_matrix(Wo, copy=True)
     bad.data[7] *= 1.01
-    assert not compare_topk_with_reference(bad, Wr, np.arange(300), 15, pair_values=pv)["ok"]
+    assert not compare_topk_with_reference(bad, Wr, np.arange(n), K, pair_values=pv)["ok"]
     # a wrong neighbour carrying the K-th value (only the exact pair evaluation can see it)
     bad = sps.lil_matrix(Wo)
     c = 11
     col = sps.csc_matrix(Wo)[:, c]
     jmin = col.indices[np.argmin(col.data)]
-    free = np.setdiff1d(np.arange(300), np.r_[col.indices, sps.csc_matrix(Wr)[:, c].indices, [c]])
+    free = np.setdiff1d(np.arange(n), np.r_[col.indices, sps.csc_matrix(Wr)[:, c].indices, [c]])
     bad[free[0], c] = col.data.min()
     bad[jmin, c] = 0
-    assert not compare_topk_with_reference(sps.csc_matrix(bad), Wr, np.arange(300), 15, pair_values=pv)["ok"]
+    assert not compare_topk_with_reference(sps.csc_matrix(bad), Wr, np.arange(n), K, pair_values=pv)["ok"]
     # a missing neighbour
     bad = sps.lil_matrix(Wo)
     bad[jmin, c] = 0
-    assert not compare_topk_with_reference(sps.csc_matrix(bad), Wr, np.arange(300), 15, pair_values=pv)["ok"]
+    assert not compare_topk_with_reference(sps.csc_matrix(bad), Wr, np.arange(n), K, pair_values=pv)["ok"]

@@ -8,6 +8,9 @@ f = 256 normal equations, multi-block Cholesky).
   configs[3]  C4-shaped rows          IALS f = 256 (user profiles ~208 like C4) + EASE_R on a 2 048-item slice at C4 density
   configs[4]  C5 1 M x 200 K, 0.05 %  ItemKNN cosine, binary: 500 columns of the benchmarked run against the compiled
                                       reference -- bitmap kernel (default) and the packed-counter window kernel
+
+The C1 and C5 ItemKNN cases also run against the reference's fp64 restatement (oracle/similarity_oracle.py), so that they
+are checked where the compiled reference is not built.
 """
 import numpy as np
 import pytest
@@ -41,23 +44,34 @@ def _against_reference(X, W, W_ref, cols):
     return res
 
 
-@pytest.mark.parametrize("values", ["binary", "ratings"])
-def test_c1_itemknn_every_column_against_the_compiled_reference(values):
+def _c1_every_column(values, reference):
     X = synth_config("C1", values=values)
     W = _sim_cls()(X, **KW).compute_similarity()
-    W_ref = _ref_cls()(X, **KW).compute_similarity()
+    W_ref = reference(X, **KW).compute_similarity()
     assert W.nnz == W_ref.nnz
     _against_reference(X, W, W_ref, np.arange(X.shape[1]))
 
 
-def test_c5_itemknn_benchmarked_kernels_against_the_compiled_reference(monkeypatch):
+@pytest.mark.parametrize("values", ["binary", "ratings"])
+def test_c1_itemknn_every_column_against_the_compiled_reference(values):
+    _c1_every_column(values, _ref_cls())
+
+
+@pytest.mark.parametrize("values", ["binary", "ratings"])
+def test_c1_itemknn_every_column_against_the_oracle(values):
+    """The same check against the fp64 restatement of the reference (oracle/similarity_oracle.py, pinned to the reference's
+    stored outputs by tests/test_oracle_similarity.py), which runs where the compiled reference is not built."""
+    _c1_every_column(values, SimilarityOracle)
+
+
+def _c5_benchmarked_kernels(monkeypatch, reference):
     """The run bench.py times (C5, binary): columns [66666, 67166) of the full-range output, produced (a) by the default
     routing (bitmap kernel K1-C, window kernel for what it hands back) and (b) by the packed 16-bit-counter window kernel
-    alone (B200REC_K1C=0), both against the reference Cython on the same URM."""
+    alone (B200REC_K1C=0), both against `reference` on the same URM."""
     X = synth_config("C5", values="binary")
     n = X.shape[1]
     lo, hi = 66666, 67166
-    W_ref = _ref_cls()(X, **KW).compute_similarity(start_col=lo, end_col=hi)
+    W_ref = reference(X, **KW).compute_similarity(start_col=lo, end_col=hi)
     Xc = sps.csc_matrix(X)
     pv = lambda jj, cc: cosine_pair_values(Xc, jj, cc, KW["shrink"])
     for k1c in ("1", "0"):
@@ -77,6 +91,15 @@ def test_c5_itemknn_benchmarked_kernels_against_the_compiled_reference(monkeypat
         assert np.array_equal(part.cnt.cpu().numpy(), cnt)
         assert np.array_equal(np.sort(part.idx.cpu().numpy(), 1), np.sort(idx, 1))
         sim._dealloc()
+
+
+def test_c5_itemknn_benchmarked_kernels_against_the_compiled_reference(monkeypatch):
+    _c5_benchmarked_kernels(monkeypatch, _ref_cls())
+
+
+def test_c5_itemknn_benchmarked_kernels_against_the_oracle(monkeypatch):
+    """The same check against the fp64 restatement of the reference, as for C1."""
+    _c5_benchmarked_kernels(monkeypatch, SimilarityOracle)
 
 
 def test_c2_slim_bpr_one_epoch_of_the_reference_recipe():
