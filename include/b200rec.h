@@ -395,6 +395,41 @@ int b200_eval_accumulate_device(const int32_t* d_users, int n_block, const int32
                                 const double* d_item_novelty, const double* d_item_pop_norm, int n_items, double* d_acc,
                                 int32_t* d_rec_count, int32_t* d_hit_count, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * K8: randomized truncated SVD (PureSVD)
+ * replaces  MatrixFactorization/PureSVDRecommender.py:36-55 -- sklearn.utils.extmath.randomized_svd(URM_train,
+ *           n_components=num_factors, random_state=random_seed) with its defaults (n_oversamples=10, n_iter='auto',
+ *           power_iteration_normalizer='auto', transpose='auto', flip_sign=True)
+ * Dense blocks are row-major fp32 [rows, ld] with ld a multiple of 4 (<= 512) and l active columns; columns l..ld-1 are zero.
+ * A (n_rows x n_cols) is the URM, or its transpose (sklearn's transpose rule: the URM when it is not wide).
+ * ------------------------------------------------------------------------------------------------ */
+/* d_Y[r, :] = sum over the stored entries (r, c, v) of the CSR matrix of v * d_X[c, :], all ld columns (the safe_sparse_dot
+ * products A @ Q and A.T @ Q of sklearn's _randomized_range_finder; A.T through the CSR of b200_csr_transpose_device) */
+int b200_csr_spmm_dense_device(int64_t n_rows, const int32_t* d_ptr, const int32_t* d_idx, const float* d_val, const float* d_X,
+                               int ld, float* d_Y, void* stream);
+/* CSR of the transpose (scipy's tocsc(): inside a column the rows ascend); d_t_ptr: n_cols + 1, d_t_idx / d_t_val: nnz */
+int b200_csr_transpose_device(int64_t n_rows, int64_t n_cols, int64_t nnz, const int32_t* d_ptr, const int32_t* d_idx,
+                              const float* d_val, int32_t* d_t_ptr, int32_t* d_t_idx, float* d_t_val, void* stream);
+/* In place: the n x l block d_Y becomes an orthonormal basis of its column span (the LU / QR normalisers of
+ * _randomized_range_finder; shifted CholeskyQR3 here).  Deficient columns are refilled with seeded Gaussian columns;
+ * *h_breakdowns (nullable) receives how many were.  l <= min(n, 512). */
+int b200_orthonormalize_device(int64_t n, int l, int ld, float* d_Y, uint32_t seed, int32_t* h_breakdowns, void* stream);
+/* _randomized_range_finder + the projection B = Q^T A of randomized_svd: from d_omega [n_cols, ld] (the Gaussian start),
+ * n_iter x (A Q, normalise, A^T Q, normalise), then d_Q [n_rows, ld] = orthonormal basis of A Q, and B^T = A^T Q = Qb Rb with
+ * d_Qb [n_cols, ld] orthonormal and d_Rb [l, l] fp64 row-major.  h_ms (nullable, 2 floats): device ms in SpMM / in
+ * orthonormalisation; h_breakdowns (nullable): deficient columns refilled over the whole call. */
+int b200_rsvd_range_device(int64_t n_rows, int64_t n_cols, const int32_t* d_ptr, const int32_t* d_idx, const float* d_val,
+                           const int32_t* d_t_ptr, const int32_t* d_t_idx, const float* d_t_val, const float* d_omega, int l, int ld,
+                           int n_iter, uint32_t seed, float* d_Q, float* d_Qb, double* d_Rb, float* h_ms, int32_t* h_breakdowns,
+                           void* stream);
+/* With svd(Rb^T) = W diag(sigma) Z^T computed on the host (h_W, h_Z: [l, l] fp64 row-major, h_sigma: the first k values):
+ * A's left factor Q W[:, :k] and right factor Qb Z[:, :k] go to d_user_factors [n_users, k] / d_item_factors [n_items, k]
+ * (swapped when `transpose`, A = URM^T), svd_flip makes the largest-magnitude entry of every user-side column positive (first
+ * row on ties), and `scale_item_side` multiplies the item-side columns by sigma (PureSVD's ITEM_factors = (diag(s) Vt)^T). */
+int b200_rsvd_finish_device(int64_t n_rows, int64_t n_cols, const float* d_Q, const float* d_Qb, int l, int ld, const double* h_W,
+                            const double* h_Z, const float* h_sigma, int k, int transpose, int scale_item_side,
+                            float* d_user_factors, float* d_item_factors, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

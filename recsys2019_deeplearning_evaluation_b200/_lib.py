@@ -103,6 +103,15 @@ SIGNATURES = {
                                                    ctypes.c_int, c_void, c_void, c_void, ctypes.c_int, c_void, c_void, c_void, c_void]),
     "b200_ials_half_epoch_device": (ctypes.c_int, [c_void, ctypes.c_int, c_void, c_void, c_void, c_void, ctypes.c_int, ctypes.c_int,
                                                    ctypes.c_double, c_void, c_void, c_void]),
+    "b200_csr_spmm_dense_device": (ctypes.c_int, [ctypes.c_int64, c_void, c_void, c_void, c_void, ctypes.c_int, c_void, c_void]),
+    "b200_csr_transpose_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, c_void, c_void, c_void, c_void, c_void,
+                                                 c_void, c_void]),
+    "b200_orthonormalize_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_void, ctypes.c_uint32, c_int_p, c_void]),
+    "b200_rsvd_range_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, c_void, c_void, c_void, c_void, c_void, c_void, c_void,
+                                              ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_uint32, c_void, c_void, c_void, c_float_p,
+                                              c_int_p, c_void]),
+    "b200_rsvd_finish_device": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, c_void, c_void, ctypes.c_int, ctypes.c_int, c_void, c_void,
+                                               c_void, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_void, c_void, c_void]),
 }
 
 _lib = None

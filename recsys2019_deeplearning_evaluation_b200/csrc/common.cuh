@@ -119,4 +119,18 @@ struct GlibcRandHost {
 
 inline unsigned div_up(long long a, long long b) { return static_cast<unsigned>((a + b - 1) / b); }
 
+// Philox4x32-10: counter = (idx, blk), key = (seed, epoch); four 32-bit words per call.
+__device__ __forceinline__ void philox_round(unsigned& c0, unsigned& c1, unsigned& c2, unsigned& c3, unsigned k0, unsigned k1) {
+  const unsigned hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+  const unsigned hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+  c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
+}
+__device__ __forceinline__ uint4 philox(unsigned long long idx, unsigned blk, unsigned seed, unsigned epoch) {
+  unsigned c0 = (unsigned)idx, c1 = (unsigned)(idx >> 32), c2 = blk, c3 = 0x9E3779B9u;
+  unsigned k0 = seed, k1 = epoch;
+#pragma unroll
+  for (int r = 0; r < 10; ++r) { philox_round(c0, c1, c2, c3, k0, k1); k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+  return make_uint4(c0, c1, c2, c3);
+}
+
 }  // namespace b200

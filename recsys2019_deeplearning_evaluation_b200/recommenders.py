@@ -9,6 +9,7 @@ follow the reference so that the evaluator and the hyper-parameter search can dr
     GraphBased/P3alphaRecommender.py:34-144, GraphBased/RP3betaRecommender.py:31-154
     SLIM_BPR/Cython/SLIM_BPR_Cython.py:67-183
     MatrixFactorization/Cython/MatrixFactorization_Cython.py:33-190
+    MatrixFactorization/PureSVDRecommender.py:20-55
     Base/Incremental_Training_Early_Stopping.py:91-261   epoch loop with periodic validation / best-model snapshot
 
 Scores, the seen-item mask and the top-`cutoff` selection run on the device (csrc/score.cu); the dense score block is
@@ -387,6 +388,27 @@ class BaseMatrixFactorizationRecommender(BaseRecommender):
         _lib.check(self._lib.b200_score_mf_device(d_users.data_ptr(), d_users.shape[0], U.data_ptr(), VT.data_ptr(), U.shape[1],
                                                   self.n_items, bu, bi, mu, out.data_ptr(), _stream()))
         return out
+
+
+class PureSVDRecommender(BaseMatrixFactorizationRecommender):
+    """MatrixFactorization/PureSVDRecommender.py:20-55: U, Sigma, VT = randomized_svd(URM_train, num_factors, random_state=
+    random_seed) on the device (rsvd.py, csrc/rsvd.cu).  Sigma goes to the item side, as the reference stores it:
+    USER_factors = U (n_users, k), ITEM_factors = (diag(Sigma) VT)^T (n_items, k), both float32, k = min(num_factors,
+    min(URM shape)).  Scores U . (Sigma VT) do not depend on that split.  random_seed=None draws the start from numpy's global
+    stream as the reference does."""
+    RECOMMENDER_NAME = "PureSVDRecommender"
+
+    def fit(self, num_factors=100, random_seed=None):
+        import torch
+        from .rsvd import rsvd_device
+        self._print("Computing SVD decomposition...")
+        r = rsvd_device(self.URM_train, num_factors, random_state=random_seed, scale_item_side=True)
+        self.USER_factors, self.ITEM_factors = r.user.cpu().numpy(), r.item.cpu().numpy()
+        # the fitted device factors go to the scorer as they are (its item side is the transpose)
+        VT = torch.empty((r.item.shape[1], r.item.shape[0]), dtype=torch.float32, device=r.item.device)
+        _lib.check(self._lib.b200_transpose_device(r.item.data_ptr(), r.item.shape[0], r.item.shape[1], VT.data_ptr(), _stream()))
+        self._d_f, self._d_f_src = (r.user, VT, None), (self.USER_factors, self.ITEM_factors)
+        self._print("... Done!")
 
 
 class _MatrixFactorization_Cython(BaseMatrixFactorizationRecommender, Incremental_Training_Early_Stopping):
